@@ -12,6 +12,9 @@ ncu launch list) against the measured tensor peak, `cpu_baseline` = the oracle t
 bench_fbo.py cases (BASELINE configs[4]), `large_batch` = the same step at 8 clips per GPU (sub-process), `clocks` =
 nvidia-smi samples taken while the timed regions ran.  N > 1 (torchrun): max over ranks, weak scaling, the N=1-only extras
 are skipped.
+
+--dump-outputs DIR writes what the last device-resident timed step computed (dump_outputs below) as DIR/<blob>.npy;
+inputs and initial weights are seeded, so two builds run with the same arguments can be compared file for file.
 """
 import argparse
 import json
@@ -20,6 +23,8 @@ import subprocess
 import sys
 import threading
 import time
+
+sys.dont_write_bytecode = True          # the benchmark writes nothing into the (possibly read-only) source tree
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 for p in (os.path.join(ROOT, 'video-long-term-feature-banks_b200', 'lib'), ROOT, os.path.join(ROOT, 'tests')):
@@ -115,6 +120,31 @@ class ClockSampler(threading.Thread):
         reasons = [n for i, n in enumerate(names) if any(s[2 + i] == 'Active' for s in self.samples)]
         return {'sm_mhz': sm[len(sm) // 2] if sm else None, 'sm_max_mhz': int(self.samples[0][1]),
                 'reasons': reasons, 'samples': len(self.samples)}
+
+
+DUMP_MAX_ELEMS = 1 << 15       # per dumped tensor: 2 x ~120 trainable tensors stay well under 64 MB of float32
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(workspace, trainable, out_dir):
+    """Write what the training step hands its caller after the last timed step, as float32 .npy files named after
+    the blobs: `loss`, the logits `pred`, and every trainable parameter after the SGD update (`<param>`) with the
+    gradient of that step (`<param>_grad`).  A tensor of more than DUMP_MAX_ELEMS elements is written as a fixed
+    sample of its flattened (logical-layout) elements: sorted indices drawn without replacement by a generator seeded
+    with the blob name, so the same elements are sampled in every run and every build."""
+    import zlib
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    names = ['loss', 'pred'] + trainable + [p + '_grad' for p in trainable]
+    total = 0
+    for n in names:
+        a = np.asarray(workspace.FetchBlob('gpu_0/' + n), dtype=np.float32)
+        if a.size > DUMP_MAX_ELEMS:
+            rng = np.random.default_rng(zlib.crc32(n.encode()))
+            a = a.reshape(-1)[np.sort(rng.choice(a.size, DUMP_MAX_ELEMS, replace=False))]
+        total += a.nbytes
+        assert total <= DUMP_MAX_BYTES, 'dumped outputs exceed %d bytes' % DUMP_MAX_BYTES
+        np.save(os.path.join(out_dir, n + '.npy'), a)
 
 
 def measured_peaks():
@@ -272,6 +302,8 @@ def run_b200(args):
     barrier()
     ms = max_over_ranks(e0.elapsed_time(e1)) / args.steps
     launches = K.LAUNCHES // max(args.steps, 1)
+    if rank == 0 and args.dump_outputs:  # before the loops below train the weights further
+        dump_outputs(workspace, model.TrainableParams(), args.dump_outputs)
 
     # ---- end to end through the public API: every step's inputs travel host (pinned) -> device inside the timed
     # region and the loss is read back every step.  EnqueueBlobs is the stand-in for the reference's BlobsQueue
@@ -472,6 +504,8 @@ def main():
     ap.add_argument('--impl', default='b200', choices=['b200', 'reference'])
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--dump-gemms', default='', help='write the per-launch GEMM table of one step here')
+    ap.add_argument('--dump-outputs', default='', metavar='DIR', help='write the outputs of the last timed step as '
+                    'DIR/<blob>.npy (loss, pred, updated parameters and their gradients; large tensors sampled)')
     ap.add_argument('--no-graph', action='store_true', help='eager launches (for ncu / debugging)')
     ap.add_argument('--no-fbo', action='store_true', help='skip the FBO-NL microbenchmark cases (bench_fbo.py)')
     ap.add_argument('--no-roofline', action='store_true', help='skip the per-launch replay profile (ncu launch lists)')
@@ -482,6 +516,10 @@ def main():
     ap.add_argument('--large-batch', type=int, default=8, help='also time the step at this many clips per GPU in a '
                     'separate process (N=1 only; 0 = skip)')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl != 'b200':
+        ap.error('--dump-outputs dumps the b200 arm')
     YAML = CONFIGS[args.config]
     CLIPS_PER_GPU = args.clips_per_gpu
     args.warmup = max(args.warmup, 3) if args.impl == 'b200' else args.warmup

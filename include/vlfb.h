@@ -86,7 +86,12 @@ typedef struct {
   int M, N, K;                /* logical GEMM extent (K per z-slice for wgrad) */
   int batch;                  /* >= 1 (DENSE only)                           */
   int taps;                   /* wgrad: number of temporal taps kT (z-slices), else 1 */
-  int split_k;                /* >= 1 (>1 needs VLFB_EPI_ATOMIC); 0 = the library picks it with the tile width */
+  int split_k;                /* >= 1 (>1 needs VLFB_EPI_ATOMIC); 0 = the library picks it with the tile width.  With
+                               * VLFB_EPI_ATOMIC, split_k == 0 and a workspace (stream_k >= 0) the product is never
+                               * split into K slices that add into d in arrival order: it runs as whole tiles or as
+                               * stream-K pieces summed in a fixed order, so the result is the same in every run.
+                               * Without a workspace, or with stream_k == -1, the library may pick plain split-K,
+                               * whose atomic additions make the last bits depend on the order the slices finish. */
   float* d;                   /* output rows: d + batch*d_batch_stride + m*ldd + n (+ tap*d_tap_stride) */
   int64_t ldd, d_batch_stride, d_tap_stride;
   float alpha;                /* applied first                               */
@@ -102,8 +107,7 @@ typedef struct {
   void* workspace;            /* stream-K scratch (partial tiles + arrival counters) of >= vlfb_gemm_workspace_bytes()
                                * bytes, 16-byte aligned, ZERO-FILLED ONCE by the caller before its first use and then
                                * only touched by vlfb_gemm (the counters are zero again when a launch ends); calls that
-                               * share it must be ordered on one stream.  NULL: stream-K is not used for non-atomic
-                               * epilogues. */
+                               * share it must be ordered on one stream.  NULL: no stream-K fix-ups (see split_k). */
   size_t workspace_bytes;
   int engine;                 /* VLFB_ENGINE_TCGEN05 (0, default) or VLFB_ENGINE_SIMT (fp32 cross-check engine) */
   int tile_n;                 /* 0 = chosen by the library, else the output-tile width (32..256, multiple of 32) */
@@ -190,6 +194,8 @@ int vlfb_avgpool3d_bwd(const float* dy, float* dx, const vlfb_conv_geom_t* g, in
 int vlfb_roi_align_fwd(const float* feat, const float* rois, float* out, int N, int H, int W,
                        int C, int R, int PH, int PW, float spatial_scale, int sampling_ratio,
                        void* stream);
+/* Backward in gather form: each element of dfeat adds the contributions of every RoI bin in a fixed order (same result
+ * in every run); PW <= 32. */
 int vlfb_roi_align_bwd(const float* dout, const float* rois, float* dfeat /* accumulated */,
                        int N, int H, int W, int C, int R, int PH, int PW, float spatial_scale,
                        int sampling_ratio, void* stream);
@@ -228,8 +234,13 @@ int vlfb_relu_bwd_tf32(const float* dy, const float* y, float* dx, int64_t n, vo
 /* out = (y == NULL || y > 0) ? round_tf32(a + b) : 0 : sum of two gradient contributions + ReLU backward + TF32
  * rounding in one pass (out may alias a or b). */
 int vlfb_add_relu_bwd_tf32(const float* a, const float* b, const float* y, float* out, int64_t n, void* stream);
-/* out[c] (+)= sum_r x[r*ld + c]  (bias gradients of Conv/FC) */
-int vlfb_colsum(const float* x, int64_t ld, float* out, int64_t rows, int cols, int accumulate, void* stream);
+/* out[c] (+)= sum_r x[r*ld + c]  (bias gradients of Conv/FC).  Slabs of rows are summed by separate CTAs and their
+ * partial sums added in slab order through `workspace` (>= vlfb_colsum_workspace_bytes(rows, cols) bytes, owned by
+ * the caller; 0 bytes: one slab), so the result is the same in every run.  Calls that share a workspace must be
+ * ordered on one stream. */
+size_t vlfb_colsum_workspace_bytes(int64_t rows, int cols);
+int vlfb_colsum(const float* x, int64_t ld, float* out, int64_t rows, int cols, int accumulate, void* workspace,
+                size_t workspace_bytes, void* stream);
 /* y = round-to-nearest TF32 of x (operand preparation for kind::tf32 MMAs; y may alias x) */
 int vlfb_round_tf32(const float* x, float* y, int64_t n, void* stream);
 int vlfb_sigmoid_fwd(const float* x, float* y, int64_t n, void* stream);

@@ -112,6 +112,13 @@ def test_gemm_plan_query():
         assert o.tile_n == 32 or N > o.tile_n // 2               # never pad N by 2x or more
         assert o.tiles == -(-M // (256 if o.pair else 128)) * -(-N // o.tile_n) * o.split_k
         assert not (o.stream_k and o.split_k != 1)
+        assert o.split_k == 1                                    # with a workspace: no order-dependent K slices
+    # conv1-style weight gradient (one tile, K ~ 8e5): stream-K pieces summed in a fixed order in the workspace; without
+    # a workspace, or with stream-K refused, plain (atomic) split-K spreads the reduction instead
+    w = plan(64, 224, 802816, split=0, flags=L.EPI_ATOMIC)
+    assert (w.split_k, w.stream_k, w.units) == (1, 1, 148)
+    assert plan(64, 224, 802816, split=0, flags=L.EPI_ATOMIC, ws=False).split_k > 1
+    assert plan(64, 224, 802816, split=0, flags=L.EPI_ATOMIC, stream_k=-1).split_k > 1
     assert lib.vlfb_gemm_plan(None, 148, None) == -1
 
 

@@ -1,7 +1,7 @@
 """2-GPU data-parallel test on the real path (SURVEY 8d config 3): one process per GPU, NCCL all-reduce of the flat
 gradient buffers, tcgen05 kernels.  After one step the replicas hold bit-identical weights, and they equal the
 single-GPU step on the concatenated batch up to the fp32 summation order of the weight gradients (one GEMM over both
-clips vs. the all-reduced sum of two).  Skipped on boxes with fewer than 2 GPUs; run with `gpurun --gpus 2`."""
+clips vs. the all-reduced sum of two).  Skipped on machines with fewer than 2 GPUs."""
 import os
 import socket
 import sys
@@ -74,7 +74,7 @@ def _worker(rank, world, port, all_inputs, params, ret):
     torch.distributed.destroy_process_group()
 
 
-@pytest.mark.skipif(torch.cuda.device_count() < 2, reason='needs 2 GPUs (gpurun --gpus 2)')
+@pytest.mark.skipif(torch.cuda.device_count() < 2, reason='needs 2 GPUs')
 def test_two_gpu_nccl_step_equals_single_gpu_step():
     import harness as H
     from oracle import model as OM

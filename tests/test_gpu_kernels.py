@@ -795,6 +795,37 @@ def test_stream_k_results_are_deterministic(K):
         _with_opts(K, {})
 
 
+
+def test_gradient_reductions_are_deterministic(K):
+    """Every reduction of the training step's backward that many CTAs share -- a weight gradient over a long K (the
+    library picks the split), a skinny long-K matmul, bias-gradient column sums and the RoIAlign backward -- gives
+    bit-identical results run after run: none of them depends on the order in which blocks finish."""
+    K.set_gemm_backend('tcgen05')
+    g = K.conv_geom((2, 8, 28, 28, 256), 256, (1, 3, 3), (1, 1, 1), (0, 1, 1))
+    x = rnd((2, 8, 28, 28, 256), 93).cuda()
+    dy = rnd(K.out_shape(g), 94).cuda()
+    a, b = rnd((1, 4, 2560), 95).cuda(), rnd((1, 2560, 80), 96).cuda()
+    rows = rnd((50000, 80), 97).cuda()
+    feat_g = rnd((4, 7, 7, 256), 98).cuda()
+    rois = torch.tensor([[0, 0., 0., 223., 223.], [1, 10.5, 20.25, 100.75, 180.5], [0, 3.3, 4.4, 30.9, 25.0],
+                         [1, 111., 7., 223., 60.]], device='cuda')
+    outs = []
+    for _ in range(3):
+        dw = torch.zeros((256, 1, 3, 3, 256), device='cuda')
+        K.conv_wgrad(dy, x, dw, g)
+        d = torch.empty((1, 4, 80), device='cuda')
+        K.matmul(a, b, d)
+        cs = torch.empty(80, device='cuda')
+        K.colsum(rows, 80, cs, 50000, 80, accumulate=False)
+        df = torch.zeros((2, 14, 14, 256), device='cuda')
+        K.roi_align_bwd(feat_g, rois, df, 1.0 / 16)
+        torch.cuda.synchronize()
+        outs.append((dw, d, cs, df))
+    for o in outs[1:]:
+        for u, v in zip(outs[0], o):
+            assert torch.equal(u, v)
+    assert outs[0][3].abs().sum() > 0 and outs[0][0].abs().sum() > 0
+
 # -------------------------------------------------------------------------- training-mode FBO-NL stack (one launch)
 def _fbo_ref(a0, bp, Ws, scale, pre_act_ln, eps=1e-5):
     """As-written NLLayers / NLCore (lfb_helper.py:170-292) in fp64 with autograd: phi and g ARE formed here."""

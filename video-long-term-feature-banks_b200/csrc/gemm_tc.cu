@@ -1792,10 +1792,23 @@ struct Plan { int bn, split_k, pair, sk; int tiles, units; double cost; };
 static constexpr bool kind_pair_capable(int kind) { return kind != VLFB_OP_STEM_K && kind != VLFB_OP_STEM_MN; }
 static constexpr bool kind_tma_capable(int) { return true; }
 
+size_t gemm_tc_workspace_bytes();
+
+// An accumulating (atomic) product whose split the library chooses is not split into K slices that add into D in
+// arrival order when the caller provides a workspace and allows stream-K: the run-to-run result would depend on that
+// order.  It runs as whole tiles or as stream-K pieces summed from the workspace in a fixed order by the last arriving
+// unit, which then adds the tile to D once.  Otherwise plain split-K (atomic, order-dependent) stays available.
+static bool det_split_of(const vlfb_gemm_params_t& p) {
+  const int want_sk = p.stream_k != 0 ? p.stream_k : env().sk;
+  return (p.flags & VLFB_EPI_ATOMIC) && p.split_k == 0 && want_sk >= 0 && p.workspace != nullptr &&
+         p.workspace_bytes >= gemm_tc_workspace_bytes();
+}
+
 // `pairs` = co-resident CTA pairs (0: pairing unavailable); pair_ok / sk_ok = what the operands / workspace allow.
 static Plan make_plan(const vlfb_gemm_params_t& p, int num_sms, int pairs, bool pair_ok, bool sk_ok) {
   const int zbase = p.taps > 1 ? p.taps : p.batch;
   const bool atomic = (p.flags & VLFB_EPI_ATOMIC) != 0;
+  const bool det_split = det_split_of(p);
   const int want_bn = p.tile_n > 0 ? p.tile_n : env().bn;
   const int want_pair = p.pair != 0 ? p.pair : env().pair;
   const int want_sk = p.stream_k != 0 ? p.stream_k : env().sk;
@@ -1824,7 +1837,7 @@ static Plan make_plan(const vlfb_gemm_params_t& p, int num_sms, int pairs, bool 
       const double cc = chunk_cost(bn, pr != 0);
       const double fixed = 8.0 * cc;
       // (a) static tile loop, optional plain split-K (atomic epilogues only)
-      const int smax = p.split_k > 0 ? p.split_k : (atomic && p.K >= 512 ? (p.K / 256 < 128 ? p.K / 256 : 128) : 1);
+      const int smax = p.split_k > 0 ? p.split_k : (atomic && !det_split && p.K >= 512 ? (p.K / 256 < 128 ? p.K / 256 : 128) : 1);
       for (int sp = (p.split_k > 0 ? p.split_k : 1); sp <= smax; ++sp) {
         const int64_t tiles = T * sp;
         const double rounds = (double)((tiles + U - 1) / U);
@@ -1836,11 +1849,13 @@ static Plan make_plan(const vlfb_gemm_params_t& p, int num_sms, int pairs, bool 
       }
       // (b) stream-K: equal chunk ranges; shared tiles reduced through the workspace (or by atomics)
       const int64_t total = T * nkt;
-      const bool sk_legal = (atomic ? p.split_k != 1 : (sk_ok && p.split_k <= 1)) && want_sk > 0 && nkt >= 2 &&
-                            total >= 2 * (int64_t)U && T * (pr ? 2 : 1) * (NEPI / 32) <= SK_CNT_INTS && U <= MAX_UNITS;
+      const bool fixup = sk_ok && (!atomic || det_split);
+      const bool sk_legal = (det_split ? sk_ok : ((atomic ? p.split_k != 1 : (sk_ok && p.split_k <= 1)) && want_sk > 0)) &&
+                            nkt >= 2 && total >= 2 * (int64_t)U && T * (pr ? 2 : 1) * (NEPI / 32) <= SK_CNT_INTS &&
+                            U <= MAX_UNITS;
       if (sk_legal && (T % U) != 0) {
         const double per_unit = (double)((total + U - 1) / U);
-        const double cost = per_unit * cc + fixed * (double)((T + U - 1) / U) + (atomic ? 1.0 : 2.0) * fixed;
+        const double cost = per_unit * cc + fixed * (double)((T + U - 1) / U) + (fixup ? 2.0 : 1.0) * fixed;
         if (cost < best_sk.cost * 0.999) {
           best_sk.cost = cost; best_sk.bn = bn; best_sk.split_k = 1; best_sk.pair = pr; best_sk.sk = 1;
           best_sk.tiles = (int)T; best_sk.units = U;
@@ -1925,6 +1940,7 @@ static int launch_variant(const cudaLaunchConfig_t& cfg, const vlfb_gemm_params_
 template <int AK, int BK, bool MASK>
 int launch(const vlfb_gemm_params_t& p_in, cudaStream_t stream) {
   vlfb_gemm_params_t p = p_in;       // split_k == 0 is resolved below
+  const bool det_split = det_split_of(p_in);
   Launch L;
   memset(&L, 0, sizeof(L));
   L.out.w = make_fastdiv(p.g.Wo);
@@ -2087,7 +2103,7 @@ int launch(const vlfb_gemm_params_t& p_in, cudaStream_t stream) {
           make_tmap_conv_flat(&tmB, p.b.ptr, g, bnh / 32))
         L.tma_b = 5;
     }
-    const bool fixup = plan.sk && !(p.flags & VLFB_EPI_ATOMIC);
+    const bool fixup = plan.sk && (!(p.flags & VLFB_EPI_ATOMIC) || det_split);
     if (!(plan.pair || fixup) || (L.tma_a && L.tma_b)) break;
     pair_ok = false;                   // an operand fell back to cp.async: plan again without pairing / fix-ups
     sk_ws = false;
@@ -2114,7 +2130,7 @@ int launch(const vlfb_gemm_params_t& p_in, cudaStream_t stream) {
     L.nkt = ceil_div(p.K, KC);
     units = cap;
     make_bounds(L.bounds, units, (int64_t)L.total_tiles, L.nkt);
-    if (!(p.flags & VLFB_EPI_ATOMIC)) {
+    if (!(p.flags & VLFB_EPI_ATOMIC) || det_split) {
       L.ws_cnt = reinterpret_cast<int*>(p.workspace);
       L.ws_tiles = reinterpret_cast<float*>(reinterpret_cast<char*>(p.workspace) + (size_t)SK_CNT_INTS * 4);
     }

@@ -260,32 +260,70 @@ __global__ void roi_align_fwd_k(const float* __restrict__ feat, const float* __r
   }
 }
 
+// Weight that the samples i = 0..g-1 of bin p along one axis (start s, bin size `bin`, extent L) give pixel P: the
+// bilinear weights of roi_sample along that axis, zero for a sample outside [-1, L].  A sample's weight at a pixel is
+// the product of its two axis weights, and it is dropped when either coordinate is out of range, so the weight of bin
+// (ph, pw) at pixel (Y, X) is axis_w(y ..., ph, Y) * axis_w(x ..., pw, X).
+__device__ __forceinline__ float roi_axis_w(float s, float bin, int g, int p, int L, int P) {
+  float t = 0.f;
+  for (int i = 0; i < g; ++i) {
+    float v = __fadd_rn(__fadd_rn(s, __fmul_rn((float)p, bin)), __fdiv_rn(__fmul_rn(__fadd_rn((float)i, 0.5f), bin), (float)g));
+    if (v < -1.0f || v > (float)L) continue;
+    if (v <= 0.f) v = 0.f;
+    int lo = (int)v, hi;
+    if (lo >= L - 1) { hi = lo = L - 1; v = (float)lo; } else hi = lo + 1;
+    const float l = __fsub_rn(v, (float)lo);
+    if (lo == P) t += __fsub_rn(1.f, l);
+    if (hi == P) t += l;
+  }
+  return t;
+}
+
+constexpr int ROI_BWD_MAX_PW = 32;     // pooled width bound of the backward (x weights of one RoI kept per thread)
+
+// dfeat += RoIAlign backward, gather form: one thread per (image, pixel, 4 channels) sums the contributions of every
+// RoI bin in a fixed order and writes its own element once -- no atomics, so the result is the same in every run.
 __global__ void roi_align_bwd_k(const float* __restrict__ dout, const float* __restrict__ rois, float* __restrict__ dfeat,
-                                int H, int W, int C, int PH, int PW, float scale, int sr, int64_t total) {
+                                int H, int W, int C, int R, int PH, int PW, float scale, int sr, int64_t total) {
   const int c4 = C >> 2;
   for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
     const int c = (int)(i % c4) * 4;
     int64_t q = i / c4;
-    const int pw = (int)(q % PW); q /= PW;
-    const int ph = (int)(q % PH); q /= PH;
-    const int r = (int)q;
-    const RoiBox b = roi_box(rois + r * 5, scale, PH, PW, sr);
-    float* f = dfeat + (int64_t)b.batch * H * W * C + c;
-    const float cnt = (float)(b.gh * b.gw);
-    float4 g = *reinterpret_cast<const float4*>(dout + i * 4);
-    g.x /= cnt; g.y /= cnt; g.z /= cnt; g.w /= cnt;
-    for (int iy = 0; iy < b.gh; ++iy)
-      for (int ix = 0; ix < b.gw; ++ix) {
-        int pos[4];
-        float w[4];
-        if (!roi_sample(b, ph, pw, iy, ix, H, W, pos, w)) continue;
-#pragma unroll
-        for (int k = 0; k < 4; ++k) {
-          float* d = f + (int64_t)pos[k] * C;
-          atomicAdd(d + 0, w[k] * g.x); atomicAdd(d + 1, w[k] * g.y);
-          atomicAdd(d + 2, w[k] * g.z); atomicAdd(d + 3, w[k] * g.w);
+    const int X = (int)(q % W); q /= W;
+    const int Y = (int)(q % H);
+    const int n = (int)(q / H);
+    float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
+    bool any = false;
+    float wxs[ROI_BWD_MAX_PW];
+    for (int r = 0; r < R; ++r) {
+      const RoiBox b = roi_box(rois + r * 5, scale, PH, PW, sr);
+      if (b.batch != n) continue;
+      const float cnt = (float)(b.gh * b.gw);
+      bool xhit = false;
+      for (int pw = 0; pw < PW; ++pw) {
+        wxs[pw] = roi_axis_w(b.x1, b.bin_w, b.gw, pw, W, X);
+        xhit |= wxs[pw] != 0.f;
+      }
+      if (!xhit) continue;
+      for (int ph = 0; ph < PH; ++ph) {
+        const float wy = roi_axis_w(b.y1, b.bin_h, b.gh, ph, H, Y);
+        if (wy == 0.f) continue;
+        for (int pw = 0; pw < PW; ++pw) {
+          const float wx = wxs[pw];
+          if (wx == 0.f) continue;
+          const float w = wy * wx / cnt;
+          const float4 g = *reinterpret_cast<const float4*>(dout + (((int64_t)r * PH + ph) * PW + pw) * C + c);
+          acc.x += w * g.x; acc.y += w * g.y; acc.z += w * g.z; acc.w += w * g.w;
+          any = true;
         }
       }
+    }
+    if (any) {
+      float4* d = reinterpret_cast<float4*>(dfeat + (((int64_t)n * H + Y) * W + X) * C + c);
+      float4 o = *d;
+      o.x += acc.x; o.y += acc.y; o.z += acc.z; o.w += acc.w;
+      *d = o;
+    }
   }
 }
 
@@ -491,25 +529,36 @@ __global__ void copy2d_k(const float* __restrict__ src, int64_t lds, float* __re
   }
 }
 
-// out[c] += sum_r x[r*ld+c]: block = 32 columns x 8 row-lanes over a slab of rows; slabs combine with
-// one atomicAdd per column (out is zeroed first unless accumulating).
+// out[c] (+)= sum_r x[r*ld+c]: block = 32 columns x 8 row-lanes over a slab of rows.  With one slab the block writes
+// out; otherwise each slab's sums go to part[slab][c] and colsum_finish_k adds the slabs in slab order, so the result
+// does not depend on the order in which blocks finish (atomics would make it differ from run to run).
 __global__ void colsum_k(const float* __restrict__ x, int64_t ld, float* __restrict__ out, int64_t rows, int cols,
-                         int64_t rows_per_block) {
-  __shared__ float part[8][33];
+                         int64_t rows_per_block, float* __restrict__ part, int accumulate) {
+  __shared__ float sp[8][33];
   const int c = blockIdx.x * 32 + threadIdx.x;
   const int64_t r0 = (int64_t)blockIdx.y * rows_per_block;
   const int64_t r1 = min(rows, r0 + rows_per_block);
   float s = 0.f;
   if (c < cols)
     for (int64_t r = r0 + threadIdx.y; r < r1; r += 8) s += x[r * ld + c];
-  part[threadIdx.y][threadIdx.x] = s;
+  sp[threadIdx.y][threadIdx.x] = s;
   __syncthreads();
   if (threadIdx.y == 0 && c < cols) {
     float t = 0.f;
 #pragma unroll
-    for (int j = 0; j < 8; ++j) t += part[j][threadIdx.x];
-    atomicAdd(out + c, t);
+    for (int j = 0; j < 8; ++j) t += sp[j][threadIdx.x];
+    if (part) part[(int64_t)blockIdx.y * cols + c] = t;
+    else out[c] = accumulate ? out[c] + t : t;
   }
+}
+
+__global__ void colsum_finish_k(const float* __restrict__ part, int slabs, float* __restrict__ out, int cols,
+                                int accumulate) {
+  const int c = blockIdx.x * blockDim.x + threadIdx.x;
+  if (c >= cols) return;
+  float t = 0.f;
+  for (int j = 0; j < slabs; ++j) t += part[(int64_t)j * cols + c];
+  out[c] = accumulate ? out[c] + t : t;
 }
 
 // ------------------------------------------------------------------ layouts
@@ -849,11 +898,12 @@ int vlfb_roi_align_fwd(const float* feat, const float* rois, float* out, int N, 
 
 int vlfb_roi_align_bwd(const float* dout, const float* rois, float* dfeat, int N, int H, int W, int C, int R, int PH,
                        int PW, float spatial_scale, int sampling_ratio, void* stream) {
-  VLFB_CHECK_ARG(dout && rois && dfeat && N > 0 && H > 0 && W > 0 && (C & 3) == 0 && R >= 0 && PH > 0 && PW > 0);
-  const int64_t total = (int64_t)R * PH * PW * (C >> 2);
-  if (total == 0) return VLFB_OK;
-  launch_k(roi_align_bwd_k, stream_grid(total, TPB), TPB, 0, ST(stream), dout, rois, dfeat, H, W, C, PH, PW, spatial_scale,
-                                                                  sampling_ratio, total);
+  VLFB_CHECK_ARG(dout && rois && dfeat && N > 0 && H > 0 && W > 0 && (C & 3) == 0 && R >= 0 && PH > 0 && PW > 0 &&
+                 PW <= ROI_BWD_MAX_PW);
+  const int64_t total = (int64_t)N * H * W * (C >> 2);
+  if (R == 0) return VLFB_OK;
+  launch_k(roi_align_bwd_k, stream_grid(total, TPB), TPB, 0, ST(stream), dout, rois, dfeat, H, W, C, R, PH, PW,
+           spatial_scale, sampling_ratio, total);
   VLFB_CHECK_LAUNCH();
   return VLFB_OK;
 }
@@ -948,23 +998,50 @@ int vlfb_add_relu_bwd_tf32(const float* a, const float* b, const float* y, float
   VLFB_CHECK_LAUNCH();
   return VLFB_OK;
 }
-int vlfb_colsum(const float* x, int64_t ld, float* out, int64_t rows, int cols, int accumulate, void* stream) {
-  VLFB_CHECK_ARG(x && out && rows >= 0 && cols > 0);
-  if (!accumulate) {
-    int rc = ew_launch<EW_FILL>(nullptr, nullptr, out, cols, 0.f, 0.f, ST(stream));
-    if (rc != VLFB_OK) return rc;
-  }
-  if (rows == 0) return VLFB_OK;
+// Row slabs of colsum: ~2 waves of 32-column blocks on 148 SMs, at least 64 rows per slab.
+static int colsum_slabs(int64_t rows, int cols) {
   const int cb = ceil_div(cols, 32);
-  int slabs = (int)((2 * 148 + cb - 1) / cb);                 // ~2 waves of blocks on 148 SMs
+  int64_t slabs = (2 * 148 + cb - 1) / cb;
   const int64_t max_slabs = (rows + 63) / 64;
-  if (slabs > max_slabs) slabs = (int)max_slabs;
-  if (slabs < 1) slabs = 1;
+  if (slabs > max_slabs) slabs = max_slabs;
+  return slabs < 1 ? 1 : (int)slabs;
+}
+
+size_t vlfb_colsum_workspace_bytes(int64_t rows, int cols) {
+  if (rows <= 0 || cols <= 0) return 0;
+  const int slabs = colsum_slabs(rows, cols);
+  return slabs > 1 ? (size_t)slabs * cols * sizeof(float) : 0;
+}
+
+int vlfb_colsum(const float* x, int64_t ld, float* out, int64_t rows, int cols, int accumulate, void* workspace,
+                size_t workspace_bytes, void* stream) {
+  VLFB_CHECK_ARG(x && out && rows >= 0 && cols > 0);
+  if (rows == 0) {
+    if (accumulate) return VLFB_OK;
+    return ew_launch<EW_FILL>(nullptr, nullptr, out, cols, 0.f, 0.f, ST(stream));
+  }
+  const int slabs = colsum_slabs(rows, cols);
+  float* part = nullptr;
+  if (slabs > 1) {
+    if (!workspace || workspace_bytes < vlfb_colsum_workspace_bytes(rows, cols)) {
+      ::vlfb::set_error("vlfb_colsum: workspace of %zu bytes < vlfb_colsum_workspace_bytes() = %zu", workspace_bytes,
+                        vlfb_colsum_workspace_bytes(rows, cols));
+      return VLFB_E_WORKSPACE;
+    }
+    part = static_cast<float*>(workspace);
+  }
   const int64_t rpb = (rows + slabs - 1) / slabs;
-  launch_k(colsum_k, dim3(cb, slabs), dim3(32, 8), 0, ST(stream), x, ld, out, rows, cols, rpb);
+  launch_k(colsum_k, dim3(ceil_div(cols, 32), slabs), dim3(32, 8), 0, ST(stream), x, ld, out, rows, cols, rpb, part,
+           accumulate);
   VLFB_CHECK_LAUNCH();
+  if (part) {
+    launch_k(colsum_finish_k, dim3(ceil_div(cols, TPB)), dim3(TPB), 0, ST(stream), (const float*)part, slabs, out, cols,
+             accumulate);
+    VLFB_CHECK_LAUNCH();
+  }
   return VLFB_OK;
 }
+
 int vlfb_sigmoid_fwd(const float* x, float* y, int64_t n, void* stream) {
   VLFB_CHECK_ARG(x && y && n >= 0);
   return ew_launch<EW_SIGMOID>(x, nullptr, y, n, 0.f, 0.f, ST(stream));

@@ -557,8 +557,11 @@ def relu_bwd_tf32(dy, y, dx):
 
 
 def colsum(x, ld, out, rows, cols, accumulate=False):
-    _check(L.load().vlfb_colsum(_ptr(x), int(ld), _ptr(out), int(rows), int(cols), int(accumulate), _stream()),
-            'colsum')
+    lib = L.load()
+    nbytes = int(lib.vlfb_colsum_workspace_bytes(int(rows), int(cols)))
+    ws = torch.empty(max(nbytes // 4, 1), dtype=torch.float32, device=out.device)     # slab partial sums
+    _check(lib.vlfb_colsum(_ptr(x), int(ld), _ptr(out), int(rows), int(cols), int(accumulate), _ptr(ws), nbytes,
+                           _stream()), 'colsum')
 
 
 def sigmoid_fwd(x, y):

@@ -95,7 +95,8 @@ SIGNATURES = {
     'vlfb_relu_bits': [_P, _P, _L, _P],
     'vlfb_relu_bwd_tf32': [_P, _P, _P, _L, _P],
     'vlfb_add_relu_bwd_tf32': [_P, _P, _P, _P, _L, _P],
-    'vlfb_colsum': [_P, _L, _P, _L, _I, _I, _P],
+    'vlfb_colsum_workspace_bytes': [_L, _I],
+    'vlfb_colsum': [_P, _L, _P, _L, _I, _I, _P, C.c_size_t, _P],
     'vlfb_sigmoid_fwd': [_P, _P, _L, _P],
     'vlfb_dropout_fwd': [_P, _P, _L, _F, _U, _U, _P, _P],
     'vlfb_copy2d': [_P, _L, _P, _L, _L, _I, _I, _P],
@@ -125,7 +126,7 @@ SIGNATURES = {
 RESTYPES = {'vlfb_last_error': C.c_char_p, 'vlfb_fbo_bank_scan_workspace': C.c_size_t,
             'vlfb_fbo_bank_scan_workspace_dt': C.c_size_t,
             'vlfb_fbo_nl_scratch_floats': C.c_size_t,
-            'vlfb_gemm_workspace_bytes': C.c_size_t, 'vlfb_spatial_bn_workspace_bytes': C.c_size_t}
+            'vlfb_gemm_workspace_bytes': C.c_size_t, 'vlfb_colsum_workspace_bytes': C.c_size_t, 'vlfb_spatial_bn_workspace_bytes': C.c_size_t}
 
 _lib = None
 
