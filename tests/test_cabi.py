@@ -122,6 +122,22 @@ def test_gemm_plan_query():
     assert lib.vlfb_gemm_plan(None, 148, None) == -1
 
 
+def test_colsum_workspace_query():
+    """Host-only: colsum needs no workspace when one slab of rows suffices (rows <= 64), else one partial sum per slab
+    and column.  Slabs: about two waves of 32-column blocks on 148 SMs, at least 64 rows each."""
+    from vlfb import libvlfb as L
+    lib = L.load()
+    for rows in (1, 63, 64, 65, 128, 129, 1000, 50000, 70000, 1 << 20):
+        for cols in (1, 20, 80, 157, 512, 2048, 9440, 9441, 20000):
+            slabs = max(1, min(-(-296 // -(-cols // 32)), -(-rows // 64)))
+            want = 0 if slabs == 1 else slabs * cols * 4
+            assert lib.vlfb_colsum_workspace_bytes(rows, cols) == want, (rows, cols)
+            if rows <= 64:
+                assert want == 0
+    assert lib.vlfb_colsum_workspace_bytes(65, 1) == 2 * 4
+    assert lib.vlfb_colsum_workspace_bytes(0, 80) == 0 and lib.vlfb_colsum_workspace_bytes(100, 0) == 0
+
+
 def test_fbo_bank_scan_split_table_properties():
     """Host-only: the split of a RoI's L bank rows over CTAs never leaves an empty split, covers all rows, and the
     workspace query matches it (csrc/fbo.cu vlfb_fbo_bank_scan_splits)."""

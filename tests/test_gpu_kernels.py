@@ -533,14 +533,22 @@ def test_losses_and_sgd(K):
     assert torch.equal(pt.cpu(), tf32_round(pd_.cpu()))
 
 
-@pytest.mark.parametrize('rows,cols', [(1200, 512), (25088, 256), (3, 80), (70000, 64)])
+@pytest.mark.parametrize('rows,cols', [(1200, 512), (25088, 256), (3, 80), (70000, 64)] +
+                         [(r, c) for r in (1, 63, 64, 65) for c in (1, 157)])
 def test_colsum(K, rows, cols):
-    x = torch.randn(rows, cols)
-    out = torch.full((cols,), 7.0, device='cuda')
-    K.colsum(x.cuda(), cols, out, rows, cols, accumulate=False)
-    assert rel_err(out, x.double().sum(0)) < 1e-5
-    K.colsum(x.cuda(), cols, out, rows, cols, accumulate=True)
-    assert rel_err(out, 2 * x.double().sum(0)) < 1e-5
+    """Dense and strided (a column block of a matrix twice as wide, ld = 2 cols) inputs, one row slab (rows <= 64)
+    and several (partial sums added in slab order); stored, then added into a random out."""
+    wide = torch.randn(rows, 2 * cols)
+    for x, ld in ((wide[:, :cols].contiguous(), cols), (wide[:, cols:], 2 * cols)):
+        s = x.double().sum(0)
+        xd = x.contiguous().cuda() if ld == cols else wide.cuda()[:, cols:]
+        out = torch.full((cols,), 7.0, device='cuda')
+        K.colsum(xd, ld, out, rows, cols, accumulate=False)
+        assert rel_err(out, s) < 1e-5, ld
+        out0 = torch.randn(cols) * float(s.abs().max())
+        out = out0.cuda()
+        K.colsum(xd, ld, out, rows, cols, accumulate=True)
+        assert rel_err(out.cpu().double() - out0.double(), s) < 1e-5, ld
 
 
 def test_weight_transpose_multi_matches_single(K):
@@ -723,6 +731,7 @@ def test_production_conv_shapes_all_tiling_variants(K, case):
     yy.backward(dy.permute(0, 4, 1, 2, 3).double())
     dx_ref = xd.grad.permute(0, 2, 3, 4, 1)
     dw_ref = wd.grad.permute(0, 2, 3, 4, 1) * s.double().view(-1, 1, 1, 1, 1)
+    dw0 = torch.randn(tuple(dw_ref.shape), generator=torch.Generator().manual_seed(80 + case)) * float(dw_ref.abs().max())
     xbits = pack_sign_bits(x)
     try:
         for opts in VARIANTS:
@@ -735,7 +744,7 @@ def test_production_conv_shapes_all_tiling_variants(K, case):
             # finishing dgrad: + residual, ReLU mask as sign bits, TF32 rounding (the epilogue of the training step)
             dxf = torch.full((2, 16, 14, 14, Ci), float('nan'), device='cuda')
             K.conv_dgrad(dy, wt, dxf, g, residual=x, relu_mask_bits=xbits, tf32_out=True)
-            dw = torch.zeros((Co,) + tuple(ker) + (Ci,), device='cuda')
+            dw = dw0.cuda()                   # accumulated: dw = pattern + row_scale * grad
             K.conv_wgrad(dy, x, dw, g, row_scale=s)
             torch.cuda.synchronize()
             assert rel_err(y, out_ref) < 2e-5, ('fwd', opts)
@@ -743,7 +752,7 @@ def test_production_conv_shapes_all_tiling_variants(K, case):
             assert rel_err(dx, dx_ref) < 2e-5, ('dgrad', opts)
             assert rel_err(dxf, (dx_ref + x.double()) * (x > 0)) < 6e-4, ('finishing dgrad', opts)
             assert (dxf[x <= 0] == 0).all() and (dxf.view(torch.int32) & 0x1FFF).eq(0).all()
-            assert rel_err(dw, dw_ref) < 2e-5, ('wgrad', opts)
+            assert rel_err(dw.double().cpu() - dw0.double(), dw_ref) < 2e-5, ('wgrad', opts)
             # the counters of the stream-K workspace are zero again after every launch
             assert int(K.gemm_workspace(x.device)[:16384].view(torch.int32).abs().sum()) == 0, opts
     finally:

@@ -153,6 +153,9 @@ int relu_bits(const float* x, uint32_t* bits, int64_t n, cudaStream_t stream);  
 int gemm_tc(const vlfb_gemm_params_t& p, cudaStream_t stream);
 void gemm_tc_plan(const vlfb_gemm_params_t& p, int num_sms, vlfb_gemm_plan_t* out);
 size_t gemm_tc_workspace_bytes();
+// True when an accumulating product must not be split into K slices that add into D in arrival order (vlfb.h,
+// split_k): the one policy both GEMM engines follow (gemm_tc.cu).
+bool gemm_fixed_order_split(const vlfb_gemm_params_t& p);
 #ifdef VLFB_TRACE
 void gemm_tc_set_trace(void* buf);
 #endif

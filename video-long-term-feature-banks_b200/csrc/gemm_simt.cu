@@ -56,7 +56,9 @@ __global__ void __launch_bounds__(256) gemm_simt_kernel(const vlfb_gemm_params_t
 
 int gemm_simt(const vlfb_gemm_params_t& p_in, cudaStream_t stream) {
   vlfb_gemm_params_t p = p_in;
-  if (p.split_k == 0) p.split_k = p.K >= 2048 ? (p.K / 1024 < 32 ? p.K / 1024 : 32) : 1;   // "library's choice"
+  // "library's choice": K slices that add into D atomically, unless the caller asked for a fixed summation order
+  if (p.split_k == 0)
+    p.split_k = gemm_fixed_order_split(p_in) ? 1 : (p.K >= 2048 ? (p.K / 1024 < 32 ? p.K / 1024 : 32) : 1);
   dim3 grid(ceil_div(p.M, TM), ceil_div(p.N, TN), (p.taps > 1 ? p.taps : p.batch) * p.split_k);
   launch_k(gemm_simt_kernel, grid, 256, 0, stream, p);
   VLFB_CHECK_LAUNCH();

@@ -1792,23 +1792,11 @@ struct Plan { int bn, split_k, pair, sk; int tiles, units; double cost; };
 static constexpr bool kind_pair_capable(int kind) { return kind != VLFB_OP_STEM_K && kind != VLFB_OP_STEM_MN; }
 static constexpr bool kind_tma_capable(int) { return true; }
 
-size_t gemm_tc_workspace_bytes();
-
-// An accumulating (atomic) product whose split the library chooses is not split into K slices that add into D in
-// arrival order when the caller provides a workspace and allows stream-K: the run-to-run result would depend on that
-// order.  It runs as whole tiles or as stream-K pieces summed from the workspace in a fixed order by the last arriving
-// unit, which then adds the tile to D once.  Otherwise plain split-K (atomic, order-dependent) stays available.
-static bool det_split_of(const vlfb_gemm_params_t& p) {
-  const int want_sk = p.stream_k != 0 ? p.stream_k : env().sk;
-  return (p.flags & VLFB_EPI_ATOMIC) && p.split_k == 0 && want_sk >= 0 && p.workspace != nullptr &&
-         p.workspace_bytes >= gemm_tc_workspace_bytes();
-}
-
 // `pairs` = co-resident CTA pairs (0: pairing unavailable); pair_ok / sk_ok = what the operands / workspace allow.
 static Plan make_plan(const vlfb_gemm_params_t& p, int num_sms, int pairs, bool pair_ok, bool sk_ok) {
   const int zbase = p.taps > 1 ? p.taps : p.batch;
   const bool atomic = (p.flags & VLFB_EPI_ATOMIC) != 0;
-  const bool det_split = det_split_of(p);
+  const bool det_split = gemm_fixed_order_split(p);
   const int want_bn = p.tile_n > 0 ? p.tile_n : env().bn;
   const int want_pair = p.pair != 0 ? p.pair : env().pair;
   const int want_sk = p.stream_k != 0 ? p.stream_k : env().sk;
@@ -1940,7 +1928,7 @@ static int launch_variant(const cudaLaunchConfig_t& cfg, const vlfb_gemm_params_
 template <int AK, int BK, bool MASK>
 int launch(const vlfb_gemm_params_t& p_in, cudaStream_t stream) {
   vlfb_gemm_params_t p = p_in;       // split_k == 0 is resolved below
-  const bool det_split = det_split_of(p_in);
+  const bool det_split = gemm_fixed_order_split(p_in);
   Launch L;
   memset(&L, 0, sizeof(L));
   L.out.w = make_fastdiv(p.g.Wo);
@@ -2179,6 +2167,16 @@ void gemm_tc_plan(const vlfb_gemm_params_t& p, int num_sms, vlfb_gemm_plan_t* ou
 }
 
 size_t gemm_tc_workspace_bytes() { return tc::gemm_tc_workspace_bytes(); }
+// An accumulating (atomic) product whose split the library chooses is not split into K slices that add into D in
+// arrival order when the caller provides a workspace and allows stream-K: the run-to-run result would depend on that
+// order.  The tensor-core engine runs it as whole tiles or as stream-K pieces summed from the workspace in a fixed
+// order by the last arriving unit, which then adds the tile to D once; the SIMT engine runs it as whole tiles.
+// Otherwise plain split-K (atomic, order-dependent) stays available.
+bool gemm_fixed_order_split(const vlfb_gemm_params_t& p) {
+  const int want_sk = p.stream_k != 0 ? p.stream_k : tc::env().sk;
+  return (p.flags & VLFB_EPI_ATOMIC) && p.split_k == 0 && want_sk >= 0 && p.workspace != nullptr &&
+         p.workspace_bytes >= gemm_tc_workspace_bytes();
+}
 #ifdef VLFB_TRACE
 void gemm_tc_set_trace(void* buf) { tc::g_trace_buf = reinterpret_cast<unsigned long long*>(buf); }
 #endif

@@ -887,7 +887,9 @@ int vlfb_avgpool3d_bwd(const float* dy, float* dx, const vlfb_conv_geom_t* g, in
 
 int vlfb_roi_align_fwd(const float* feat, const float* rois, float* out, int N, int H, int W, int C, int R, int PH,
                        int PW, float spatial_scale, int sampling_ratio, void* stream) {
-  VLFB_CHECK_ARG(feat && rois && out && N > 0 && H > 0 && W > 0 && (C & 3) == 0 && R >= 0 && PH > 0 && PW > 0);
+  // R == 0 (a batch without boxes) is a no-op: empty rois / out buffers may then be null
+  VLFB_CHECK_ARG(feat && (R == 0 || (rois && out)) && N > 0 && H > 0 && W > 0 && (C & 3) == 0 && R >= 0 && PH > 0 &&
+                 PW > 0);
   const int64_t total = (int64_t)R * PH * PW * (C >> 2);
   if (total == 0) return VLFB_OK;
   launch_k(roi_align_fwd_k, stream_grid(total, TPB), TPB, 0, ST(stream), feat, rois, out, H, W, C, PH, PW, spatial_scale,
@@ -898,8 +900,8 @@ int vlfb_roi_align_fwd(const float* feat, const float* rois, float* out, int N, 
 
 int vlfb_roi_align_bwd(const float* dout, const float* rois, float* dfeat, int N, int H, int W, int C, int R, int PH,
                        int PW, float spatial_scale, int sampling_ratio, void* stream) {
-  VLFB_CHECK_ARG(dout && rois && dfeat && N > 0 && H > 0 && W > 0 && (C & 3) == 0 && R >= 0 && PH > 0 && PW > 0 &&
-                 PW <= ROI_BWD_MAX_PW);
+  VLFB_CHECK_ARG((R == 0 || (dout && rois)) && dfeat && N > 0 && H > 0 && W > 0 && (C & 3) == 0 && R >= 0 && PH > 0 &&
+                 PW > 0 && PW <= ROI_BWD_MAX_PW);
   const int64_t total = (int64_t)N * H * W * (C >> 2);
   if (R == 0) return VLFB_OK;
   launch_k(roi_align_bwd_k, stream_grid(total, TPB), TPB, 0, ST(stream), dout, rois, dfeat, H, W, C, R, PH, PW,
